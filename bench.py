@@ -2,6 +2,7 @@
 """bench.py -- FNO rollout steps/sec on 64x64 cavity fields (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--act bf16|f32]
+                    [--dump-outputs DIR]
 
 One "step" = one `generate()` of the whole per-GPU batch (one autoregressive rollout step,
 SURVEY.md 8d).  N=1 workload = BASELINE.json configs[1]: cavity (p=5), batch 256, hidden activations
@@ -14,6 +15,10 @@ the timed region every step), "roofline" (dominant kernel, algorithmic bytes / C
 measured HBM peak), "kernels" (per-kernel mean durations from a second, event-bracketed pass),
 "cpu_baseline" (oracle torch port = the reference's own library calls, timed on this host's cores),
 "rel_l2" (per-step relative L2 vs the fp32 CPU oracle on identical inputs) and "clocks".
+
+--dump-outputs DIR writes what the timed rollout returned for its last step, for both storage modes, as
+DIR/preds_last_step_{bf16,f32}.npy (float32, B x 2 x 64 x 64; rank 0's shard).  Weights and inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -309,10 +314,10 @@ def host_cpu():
 
 def reference_impl(sd):
     """The CPU implementation `cpu_baseline` / `--impl reference` time, as (kind, forward, train_step_factory).
-    kind "reference": the UNMODIFIED reference module, installed by __graft_entry__.build() from /root/reference/src into
-    the git-ignored baseline/_ref/ (it travels to the GPU box with the snapshot); kind "port": oracle/fno_torch_port.py,
-    verified bit-identical to it by oracle/make_golden.py, when baseline/_ref is absent."""
-    ref_src = os.path.join(ROOT, "baseline", "_ref", "src")
+    kind "reference": the UNMODIFIED reference module, byte-compiled by __graft_entry__.build() into the git-ignored
+    oracle/_ref/src (oracle/build_ref.py); kind "port": oracle/fno_torch_port.py, verified bit-identical to it by
+    oracle/make_golden.py, when oracle/_ref is absent."""
+    ref_src = os.path.join(ROOT, "oracle", "_ref", "src")
     if os.path.isdir(os.path.join(ref_src, "models", "fno")):
         try:
             sys.path.insert(0, ref_src)
@@ -344,7 +349,7 @@ def reference_impl(sd):
                 return step
             return "reference", fwd, many, make_train
         except Exception as e:  # noqa: BLE001
-            sys.stderr.write(f"bench.py: baseline/_ref unusable ({type(e).__name__}: {e}); timing the oracle port\n")
+            sys.stderr.write(f"bench.py: oracle/_ref unusable ({type(e).__name__}: {e}); timing the oracle port\n")
         finally:
             if sys.path and sys.path[0] == ref_src:
                 sys.path.pop(0)
@@ -416,14 +421,27 @@ def cpu_baseline(sd, batch, budget_s: float = 12.0, max_steps: int = 6):
     return out
 
 
+def dump_outputs(out_dir: str, arrays: dict, limit: int = 64 << 20) -> None:
+    """Write every (B, ...) array as out_dir/<name>.npy in float32.  When they would exceed `limit` bytes together, each
+    keeps the batch rows np.random.default_rng(0) picks (sorted), the same rows in every run with the same --batch."""
+    os.makedirs(out_dir, exist_ok=True)
+    budget = limit // max(len(arrays), 1)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        rows = max(budget // (a[0].nbytes or 1), 1)
+        if rows < a.shape[0]:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], rows, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def workload_name(batch: int) -> str:
     return (f"FNO autoregressive rollout, cavity_prop_bc_geo shape (p=5), batch {batch}/GPU, 64x64x2 "
             f"fields, 4 Fourier layers x 32 ch x 12x12 modes (BASELINE.json configs[1])")
 
 
 def run_reference(args, rank: int, world: int):
-    """--impl reference: the reference's own CPU implementation of the path (the unmodified module from baseline/_ref when
-    build() could install it, else the verified port) on ALL physical cores of this host -- also under torchrun, where
+    """--impl reference: the reference's own CPU implementation of the path (the unmodified module from oracle/_ref when
+    build() could compile it, else the verified port) on ALL physical cores of this host -- also under torchrun, where
     OMP_NUM_THREADS=1 would otherwise leave it single-threaded.  Rank 0 only; the other ranks exit."""
     if rank != 0:
         return
@@ -451,7 +469,7 @@ def run_reference(args, rank: int, world: int):
         # same workload as the GPU arm; one step = one pass over one batch of `batch_per_gpu` cases
         "config": {"workload": workload_name(args.batch), "batch_per_gpu": args.batch, "global_batch": args.batch,
                    "act_storage": "f32", "arithmetic": "fp32",
-                   "implementation": (f"reference CPU path ({'unmodified src/models/fno/fno2d.py from baseline/_ref' if kind == 'reference' else 'torch port of src/models/fno/fno2d.py'}), "
+                   "implementation": (f"reference CPU path ({'unmodified src/models/fno/fno2d.py from oracle/_ref' if kind == 'reference' else 'torch port of src/models/fno/fno2d.py'}), "
                                       f"{threads} threads on {cpu_model} ({phys} cores), rank 0 only")},
         "sample_steps_per_s": val * args.batch,
         "cpu_baseline": {"value": val, "unit": UNIT, "cores": threads, "kind": kind, "cpu_model": cpu_model,
@@ -473,7 +491,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true",
                     help="launch every kernel on the stream instead of replaying the rollout from a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the predictions of the last timed rollout step of each storage mode as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -491,7 +513,7 @@ def main():
     batch = synth.make_batch(1 + rank, args.batch, "cavity", with_label=False)  # seed 0(+rank) shards (SURVEY 8d)
     inp, cp, mk = (torch.from_numpy(batch[k]).to(dev) for k in ("inputs", "case_params", "mask"))
 
-    results = {}
+    results, last_preds = {}, {}
     sampler = ClockSampler(local)
     for act in ([args.act] + [a for a in ("bf16", "f32") if a != args.act]):
         model, sd = build_model(act, p)
@@ -499,9 +521,12 @@ def main():
         headline = act == args.act
         if headline and rank == 0:
             sampler.start()
-        ts, _ = timed_rollout(model, inp, cp, mk, args.steps, args.warmup, reps=5 if headline else 3)
+        ts, seq = timed_rollout(model, inp, cp, mk, args.steps, args.warmup, reps=5 if headline else 3)
         if headline and rank == 0:
             clocks = sampler.stop()
+        if args.dump_outputs and rank == 0:
+            last_preds[act] = seq[-1].cpu()   # a copy: seq[-1] is a view of the whole K-step rollout tensor
+        del seq
         ts_max = [dp.max_over_ranks(t, dev) for t in ts]   # max over ranks of every repetition
         r = {"t": float(np.median(ts_max)), "t_min": float(min(ts_max)), "t_all": ts_max}
         if headline:
@@ -526,6 +551,8 @@ def main():
         if torch.distributed.is_initialized():
             torch.distributed.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {f"preds_last_step_{a}": t for a, t in last_preds.items()})
 
     peak, peak_src = measured_hbm_peak()
 

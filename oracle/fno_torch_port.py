@@ -1,8 +1,8 @@
 """TEST INFRASTRUCTURE -- CPU PyTorch restatement ("port") of the reference FNO hot path.
 
 Never imported by the product package; only `tests/`, `__graft_entry__.smoke()` and the
-`cpu_baseline` / `--impl reference` legs of `bench.py` may use it (the reference itself lives in
-/root/reference, which does not exist on the GPU box, so this port is what gets timed there).
+`cpu_baseline` / `--impl reference` legs of `bench.py` may use it (the reference is not part of this
+repository, so this port is what those legs time).
 
 It issues the *same library calls* the reference issues on CPU, so its speed is the reference's:
 torch.fft.rfft2 -> zero-filled cfloat spectrum -> two einsum("bixy,ioxy->boxy") corner products ->

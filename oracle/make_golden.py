@@ -1,8 +1,8 @@
 """TEST INFRASTRUCTURE -- generate tests/golden/*.npz from the UNMODIFIED reference module.
 
-Run in the build container only (needs /root/reference):
+Needs an unmodified CFDBench `src/` tree: CFDBENCH_SRC, else oracle/build_ref.py's default location:
 
-    PYTHONDONTWRITEBYTECODE=1 python oracle/make_golden.py
+    CFDBENCH_SRC=/path/to/CFDBench/src PYTHONDONTWRITEBYTECODE=1 python oracle/make_golden.py
 
 For each case it (1) builds the reference `Fno2d` (reference src/models/fno/fno2d.py:115) with
 weights from `cfdbench_b200.synth.make_state_dict(seed)` loaded through `load_state_dict`,
@@ -20,7 +20,9 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, "/root/reference/src")
+from oracle import build_ref  # noqa: E402
+
+sys.path.insert(0, build_ref.source_dir())
 sys.dont_write_bytecode = True
 
 from models.fno.fno2d import Fno2d, SpectralConv2d_fast  # noqa: E402  (the reference)
@@ -33,11 +35,13 @@ from oracle import fno_torch_port as opt  # noqa: E402
 GOLD = os.path.join(ROOT, "tests", "golden")
 
 CASES = [
-    # name, problem, batch, weight seed, batch seed, spectral gain, rollout steps
-    ("cavity_b2_gain200", "cavity", 2, 101, 201, 200.0, 3),
-    ("cylinder_b2_gain200", "cylinder", 2, 102, 202, 200.0, 3),
-    ("cavity_b1_default_init", "cavity", 1, 103, 203, 1.0, 20),
+    # name, problem, batch, weight seed, batch seed, spectral gain, rollout steps, spectral weight gradients stored
+    ("cavity_b2_gain200", "cavity", 2, 101, 201, 200.0, 3, False),
+    ("cylinder_b2_gain200", "cylinder", 2, 102, 202, 200.0, 3, True),
+    ("cavity_b1_default_init", "cavity", 1, 103, 203, 1.0, 20, False),
 ]
+# hidden activations are stored for these channels only, which keeps every fixture under 1 MB
+ACT_CHANNELS = np.arange(0, synth.HIDDEN, 8)
 
 
 def ref_model(sd: dict, p: int) -> Fno2d:
@@ -50,7 +54,7 @@ def ref_model(sd: dict, p: int) -> Fno2d:
 def main() -> None:
     torch.set_num_threads(8)
     os.makedirs(GOLD, exist_ok=True)
-    for name, problem, b, wseed, bseed, gain, steps in CASES:
+    for name, problem, b, wseed, bseed, gain, steps, spectral_grads in CASES:
         p = synth.n_case_params(problem)
         sd = synth.make_state_dict(wseed, n_params=p, spectral_gain=gain)
         batch = synth.make_batch(bseed, b, problem)
@@ -109,14 +113,15 @@ def main() -> None:
             preds=out["preds"].detach().numpy(),
             loss=np.array([out["loss"][k].item() for k in ("mse", "rmse", "mae", "nmse")], dtype=np.float64),
             rollout=np.stack([r.numpy() for r in roll]),
-            act0_b0=acts[0][:1], act1_b0=acts[1][:1], act4_b0=acts[-1][:1],
-            spectral0_b0=spec[:1],
+            act_channels=ACT_CHANNELS,
+            act0_b0=acts[0][:1, ACT_CHANNELS], act1_b0=acts[1][:1, ACT_CHANNELS], act4_b0=acts[-1][:1, ACT_CHANNELS],
+            spectral0_b0=spec[:1, ACT_CHANNELS],
         )
         for k in ("fc0.weight", "fc0.bias", "fc1.weight", "fc1.bias", "fc2.weight", "fc2.bias",
                   "blocks.0.w0.weight", "blocks.0.w0.bias", "blocks.3.w0.weight", "blocks.3.w0.bias"):
             store["grad::" + k] = grads[k]
         for k in ("blocks.0.conv0.weights1", "blocks.0.conv0.weights2", "blocks.3.conv0.weights1",
-                  "blocks.3.conv0.weights2"):
+                  "blocks.3.conv0.weights2") if spectral_grads else ():
             store["gradslice::" + k] = grads[k][:, :, ::4, ::4]           # (32,32,3,3) complex
             store["gradnorm::" + k] = np.array(np.linalg.norm(grads[k]))
         np.savez_compressed(os.path.join(GOLD, name + ".npz"), **store)

@@ -1,7 +1,8 @@
 """The reference's own scripts, UNCHANGED, on the drop-in (north_star: "train_auto.py and test_multistep.py run unchanged").
 
-`baseline/_ref/src` is the unmodified reference tree copied by `__graft_entry__.build()` (git-ignored, travels to the GPU
-box with the snapshot).  `python -m cfdbench_b200.runner <src> <script> --stub-missing ...` rebinds the plug-in seam
+The scripts come from `oracle/_ref/src`, the unmodified reference tree byte-compiled there by `__graft_entry__.build()`
+(oracle/build_ref.py), or from a CFDBench `src/` directory named by CFDBENCH_SRC; the tests skip when neither exists.
+`python -m cfdbench_b200.runner <src> <script> --stub-missing ...` rebinds the plug-in seam
 (reference src/utils/autoregressive.py:10) and runs the script as `__main__`; stand-ins are installed only for packages
 this image lacks (tap, matplotlib, diffusers, ...).  Data: a tiny on-disk cavity set in the reference's format
 (tools/make_tiny_cavity.py; reference src/dataset/cavity.py:15-34).
@@ -19,16 +20,18 @@ import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_SRC = os.path.join(ROOT, "baseline", "_ref", "src")
+REF_SRC = os.path.abspath(os.environ.get("CFDBENCH_SRC") or os.path.join(ROOT, "oracle", "_ref", "src"))
 
 pytestmark = [pytest.mark.gpu,
               pytest.mark.skipif(not os.path.isdir(os.path.join(REF_SRC, "models", "fno")),
-                                 reason="baseline/_ref/src (installed by __graft_entry__.build()) is not present")]
+                                 reason="no reference tree: oracle/_ref/src was not built and CFDBENCH_SRC is unset")]
 
 COMMON = ["--model", "fno", "--data_name", "cavity_prop_bc_geo", "--loss_name", "nmse", "--lr", "0.001"]
 
 
 def run_script(script, data_dir, out_dir, extra, act=None):
+    if not os.path.exists(os.path.join(REF_SRC, script)):
+        script += "c"   # the byte-compiled tree holds train_auto.pyc, ...
     cmd = [sys.executable, "-m", "cfdbench_b200.runner", REF_SRC, script, "--stub-missing"]
     if act:
         cmd += ["--act-dtype", act]

@@ -315,12 +315,29 @@ def test_bench_reference_arm_prints_one_contract_line():
         assert key in d, key
     assert d["impl"] == "reference" and d["metric"] == "fno_rollout_steps_per_sec" and d["unit"] == "steps/s"
     assert d["higher_is_better"] is True and d["gpu_launches"] == 0 and d["value"] > 0
-    ref_installed = os.path.isdir(os.path.join(ROOT, "baseline", "_ref", "src", "models", "fno"))
-    assert d["cpu_baseline"]["kind"] == ("reference" if ref_installed else "port") and d["cpu_baseline"]["cores"] >= 1
+    ref_built = os.path.isdir(os.path.join(ROOT, "oracle", "_ref", "src", "models", "fno"))
+    assert d["cpu_baseline"]["kind"] == ("reference" if ref_built else "port") and d["cpu_baseline"]["cores"] >= 1
     assert d["cpu_baseline"]["cpu_model"]
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
     import bench
     assert d["config"]["workload"] == bench.workload_name(2)
+
+
+def test_bench_dump_outputs_writes_float32_within_the_limit(tmp_path):
+    """bench.py --dump-outputs: one float32 .npy per array; over the byte limit, the same seeded batch rows every time."""
+    import bench
+    a = torch.arange(8 * 2 * 4 * 4, dtype=torch.float32).reshape(8, 2, 4, 4)
+    bench.dump_outputs(str(tmp_path / "full"), {"x": a})
+    np.testing.assert_array_equal(np.load(tmp_path / "full" / "x.npy"), a.numpy())
+    limit = 2 * 3 * a[0].numel() * 4   # two arrays, three rows each
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), {"x": a, "y": a.double()}, limit=limit)
+    x1, y1, x2 = (np.load(tmp_path / d / f"{n}.npy") for d, n in (("s1", "x"), ("s1", "y"), ("s2", "x")))
+    assert x1.dtype == y1.dtype == np.float32 and x1.shape == (3, 2, 4, 4) and x1.nbytes + y1.nbytes <= limit
+    np.testing.assert_array_equal(x1, x2)
+    rows = x1[:, 0, 0, 0].astype(int) // a[0].numel()
+    np.testing.assert_array_equal(x1, a.numpy()[rows])
+    assert list(rows) == sorted(set(rows))
 
 
 def test_bench_train_line_names_the_allreduce_mode():
